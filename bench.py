@@ -2,7 +2,7 @@
 """bench.py -- agent*steps/sec of the GCBF train step (one inner iteration of GCBF.update, reference
 gcbf/algo/gcbf.py:158-226) on synthetic BASELINE.json configs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C3] [--also C2,...|none] [--impl own|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C3] [--also C2,...|none] [--impl own|reference] [--dump-outputs DIR]
 
 Workload     : `value` / `e2e` / `roofline` are measured on --config, by default C3 (DubinsCar n=1024, obs=32, B=64 per GPU) -- the
                largest single-GPU configuration of BASELINE.json.  `config.also` carries the same device-timed and end-to-end
@@ -16,6 +16,11 @@ own arm      : gcbf_b200 (sm_100a kernels through the C ABI).  `value` = device-
 reference arm: the reference algorithm on the host CPU cores.  The reference is pure Python on torch_geometric, which
                cannot be installed on the GPU box, so this arm times oracle/gcbf_oracle.py (a port validated
                bit-for-bit against the reference in the build container) -- kind "port".
+Outputs      : --dump-outputs DIR writes what the last timed step of --config handed its caller (rank 0's share) as DIR/<name>.npy,
+               see step_outputs().  That step starts from the seeded weights and optimiser state (restored before it, outside the
+               timed interval), so the same arguments give the same inputs on every run and two builds can be compared output for
+               output: the weight-gradient reductions add in a run-dependent order, and clipped Adam grows those last-bit
+               differences into visibly different weights within a few steps.
 Multi-GPU    : one process per GPU (torchrun), environment-parallel: every rank trains on its own B graphs (weak
                scaling), one NCCL all-reduce of the flat gradient bucket per step.
 Prints ONE JSON line on rank 0.
@@ -147,8 +152,46 @@ def build_case(cfg_name, device, rank):
     return sb, env, algo
 
 
-def measure(cfg_name, args, dev, rank, world, dist, with_roofline, sampler=None):
-    """Device-timed and end-to-end throughput of one BASELINE config on this rank's share (max over ranks taken by the caller)."""
+DUMP_MAX_ELEMS = 1 << 20        # per array: larger outputs are dumped as a fixed, seeded sample (all arrays together stay under 64 MB)
+
+
+def step_outputs(res, algo):
+    """What one train step hands its caller, copied to the host before the next step reuses the step's workspace: every tensor of
+    the result dict (integer / float64 tensors as float64, the rest as float32) and the updated parameters (the flat bucket).
+    An array of more than DUMP_MAX_ELEMS elements is replaced by the elements at a fixed, seeded, sorted set of flat indices."""
+    arrays = dict(res, params=algo._bucket.flat)
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        t = t.cpu()
+        out[name] = (t.double() if t.dtype in (torch.int32, torch.int64, torch.float64) else t.float()).numpy()
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    return out
+
+
+def train_state(algo):
+    """Copies of everything a train step reads and rewrites: parameters, spectral-norm vectors, Adam moments and step count."""
+    b = algo._ensure_bucket()
+    return ([{k: v.clone() for k, v in m.state_dict().items()} for m in (algo.cbf, algo.actor)], b.exp_avg.clone(),
+            b.exp_avg_sq.clone(), b.step)
+
+
+def restore_train_state(algo, state):
+    sds, exp_avg, exp_avg_sq, step = state
+    for m, sd in zip((algo.cbf, algo.actor), sds):
+        m.load_state_dict(sd)          # in-place copies: the library sees new weight versions and refreshes its fp16 companions
+    b = algo._bucket
+    b.exp_avg.copy_(exp_avg)
+    b.exp_avg_sq.copy_(exp_avg_sq)
+    b.step = step
+
+
+def measure(cfg_name, args, dev, rank, world, dist, with_roofline, sampler=None, dump=False):
+    """Device-timed and end-to-end throughput of one BASELINE config on this rank's share (max over ranks taken by the caller).
+    With `dump`, the last timed step starts from the seeded state and its outputs are returned (step_outputs)."""
     from gcbf_b200 import _C, ops
     sb, env, algo = build_case(cfg_name, dev, rank)
     algo.process_group = None
@@ -161,6 +204,7 @@ def measure(cfg_name, args, dev, rank, world, dist, with_roofline, sampler=None)
             dist.barrier()
         torch.cuda.synchronize()
 
+    seeded = train_state(algo) if dump else None
     # ---- device-timed region: batch resident in HBM ---------------------------------------------------------
     for _ in range(args.warmup):
         algo.train_step(data)
@@ -169,16 +213,22 @@ def measure(cfg_name, args, dev, rank, world, dist, with_roofline, sampler=None)
         sampler.start()
     _C.reset_counters()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    pause0, pause1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
-    for _ in range(args.steps):
+    for i in range(args.steps):
+        if seeded is not None and i == args.steps - 1:
+            pause0.record()
+            restore_train_state(algo, seeded)
+            pause1.record()
         res = algo.train_step(data)
     ev1.record()
     barrier()
-    ms = ev0.elapsed_time(ev1)
+    ms = ev0.elapsed_time(ev1) - (pause0.elapsed_time(pause1) if seeded is not None else 0.0)
     launches = _C.kernel_launches()
     clocks = sampler.stop() if sampler is not None else None
     scal = res['scalars'].tolist()
+    outputs = step_outputs(res, algo) if dump else None
     # ---- end-to-end: host buffers in, scalars out, every step ---------------------------------------------------
     host_states = sb.states.pin_memory()
     h2d = host_states.numel() * 4
@@ -244,7 +294,7 @@ def measure(cfg_name, args, dev, rank, world, dist, with_roofline, sampler=None)
         dist.all_reduce(et)
     del algo, data
     return dict(sb=sb, B=B, n=n, E=E, E_total=int(et.item()), ms=ms, ms_e2e=ms_e2e, e2e_runs=e2e_runs, h2d=h2d, launches=launches, clocks=clocks,
-                scal=scal, gemm=gemm, ms_instr=ms_instr)
+                scal=scal, gemm=gemm, ms_instr=ms_instr, outputs=outputs)
 
 
 def rollout_leg(cfg_name, dev, steps=20):
@@ -330,7 +380,7 @@ def run_own(args):
 
     gpu_leg_threads()
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    m = measure(main_cfg, args, dev, rank, world, dist, True, sampler)
+    m = measure(main_cfg, args, dev, rank, world, dist, True, sampler, dump=args.dump_outputs is not None)
     extra = {}
     for c in also:
         if world == 1:
@@ -416,6 +466,11 @@ def run_own(args):
             line['rollout'] = {'error': repr(ex)[:200]}
     if world == 1 and not args.no_cpu_baseline:
         line['cpu_baseline'] = cpu_baseline(main_cfg, budget_s=25.0)
+    if args.dump_outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in m['outputs'].items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -558,7 +613,7 @@ def run_macbf(args):
     dev = torch.device('cuda', 0)
     out = {}
     for name in macbf_probe.WORKLOADS:
-        rec, (sb, algo, data) = macbf_probe.measure(name, dev, steps=max(args.steps, 10), warmup=max(args.warmup, 3))
+        rec, (sb, algo, data) = macbf_probe.measure(name, dev, steps=args.steps, warmup=args.warmup)
         if name == 'ref' and not args.no_cpu_baseline:
             host_threads()
             sys.path.insert(0, os.path.join(ROOT, 'oracle'))
@@ -592,7 +647,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true', help='skip the host-buffer leg (profiling runs under ncu only)')
     ap.add_argument('--macbf', action='store_true', help='measure the MACBF baseline train step instead (SURVEY 8f-4; single GPU, own arm only)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed train step of --config as DIR/<name>.npy (own arm, GCBF only)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs is not None and (args.impl != 'own' or args.macbf):
+        ap.error('--dump-outputs writes the outputs of the GCBF train step of the own arm (not with --impl reference or --macbf)')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -4,6 +4,7 @@ gcbf_b200/synth.py and a seeded module construction, so the fixtures hold only o
 
     python oracle/make_golden.py            # regenerate every GCBF case
     python oracle/make_golden.py macbf      # regenerate the MACBF cases (tests/golden/macbf_*.pt)
+    python oracle/make_golden.py live       # regenerate tests/golden/reference_runs.json
 """
 import os
 import sys
@@ -33,11 +34,23 @@ MACBF_CASES = {
 }
 INIT_SEED = 0
 STEPS = 2
+# intra-op threads of every fixture run: MKL's QR inside the seeded orthogonal_ initialisation rounds differently at other thread
+# counts, so tests/test_oracle_cpu.py runs the port at this count too
+THREADS = 8
+# one train step from seed 5, compared bit for bit (tests/test_oracle_cpu.py::test_port_matches_live_reference); the post-step
+# state dicts are stored as per-tensor SHA-256 of their float32 bytes, which keeps the comparison exact at a few kB
+LIVE_CASES = [('SimpleCar', 12, 0, 2, 2.0), ('DubinsCar', 10, 3, 2, 2.0), ('SimpleDrone', 6, 6, 2, 1.0)]
+LIVE_SEED = 5
 
 
 def digest(sd):
     return {k: dict(sum=float(v.double().sum()), abssum=float(v.double().abs().sum()),
                     head=v.reshape(-1)[:4].clone()) for k, v in sd.items()}
+
+
+def sha256(t):
+    import hashlib
+    return hashlib.sha256(t.detach().cpu().contiguous().numpy().tobytes()).hexdigest()
 
 
 def main():
@@ -88,8 +101,56 @@ def main_macbf():
               f'safe={int(res["safe_mask"].sum())} loss_hdot={s["loss/derivative"]:.6f} -> {os.path.getsize(path)} B')
 
 
+def reference_buffer_sampling():
+    """The reference's replay buffer (gcbf/algo/buffer.py): appends, seeded segment sampling (balanced and not), a merge."""
+    import random
+    import numpy as np
+    from ref_loader import load_reference
+    load_reference()
+    from gcbf.algo.buffer import Buffer
+    buf, other = Buffer(), Buffer()
+    for i in range(90):
+        buf.append(i, i % 4 != 0)
+    for i in range(200, 230):
+        other.append(i, i % 3 == 0)
+    out = []
+    for seed, (n, m, bal) in enumerate([(12, 3, False), (16, 3, True), (7, 1, False), (20, 5, True)]):
+        np.random.seed(seed)
+        random.seed(seed)
+        out.append(buf.sample(n, m, bal))
+    buf.merge(other)
+    np.random.seed(9)
+    random.seed(9)
+    out.append(buf.sample(24, 3, True))
+    out.append([buf.size, buf.safe_data[-3:], buf.unsafe_data[-3:]])
+    return out
+
+
+def main_live():
+    """tests/golden/reference_runs.json: what the CPU tests compare the port and the replay buffers against."""
+    import json
+    synth = ref_harness._load_synth()
+    cases = []
+    for env_name, n, obs, graphs, area in LIVE_CASES:
+        sb = synth.make_states(env_name, n, obs, graphs, area, LIVE_SEED)
+        res = ref_harness.run_reference(sb, 0, None, 1)
+        cases.append(dict(env=env_name, n=n, obs=obs, graphs=graphs, area=area, seed=LIVE_SEED,
+                          edge_index=res['edge_index'].tolist(), h_probe=res['h_probe'].tolist(), u_probe=res['u_probe'].tolist(),
+                          cbf_final_sha256={k: sha256(v) for k, v in res['cbf_final'].items()},
+                          actor_final_sha256={k: sha256(v) for k, v in res['actor_final'].items()}))
+        print(f'{env_name}: E={res["edge_index"].shape[1]} agents={res["h_probe"].shape[0]}')
+    path = os.path.join(os.path.dirname(HERE), 'tests', 'golden', 'reference_runs.json')
+    with open(path, 'w') as f:
+        json.dump(dict(train_step=cases, buffer_sampling=reference_buffer_sampling()), f, indent=1)
+        f.write('\n')
+    print(f'{path}: {os.path.getsize(path)} B')
+
+
 if __name__ == '__main__':
+    torch.set_num_threads(THREADS)
     if len(sys.argv) > 1 and sys.argv[1] == 'macbf':
         main_macbf()
+    elif len(sys.argv) > 1 and sys.argv[1] == 'live':
+        main_live()
     else:
         main()

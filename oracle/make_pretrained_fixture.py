@@ -9,10 +9,13 @@ Writes
   tests/golden/pretrained_stats.pt          per-tensor statistics of all six checkpoints (shape, mean, std, absmax, row-norm range,
                                             quantiles) -- lets a test synthesise "trained-like" weights where the 98 MB files
                                             are absent
+  tests/golden/pretrained_checkpoints.json  layout of all six checkpoint files (key order, shapes, state-dict metadata, file size)
+                                            -- lets a test write checkpoints the shipped files' shape without their weights
   tests/golden/_pretrained/<env>/*.pkl      a byte copy of the checkpoint files for ONE env (git-ignored: weights are data, not
                                             history; the directory travels to the GPU box with the working tree)
 
     python oracle/make_pretrained_fixture.py
+    python oracle/make_pretrained_fixture.py manifest     # only tests/golden/pretrained_checkpoints.json
 """
 import os
 import shutil
@@ -76,7 +79,30 @@ def main():
                 shutil.copyfile(os.path.join(ckpt, f), os.path.join(dst, f))
                 os.chmod(os.path.join(dst, f), 0o644)
     torch.save(stats, os.path.join(out_dir, 'pretrained_stats.pt'))
+    checkpoint_manifest()
+
+
+def checkpoint_manifest():
+    import json
+    out = {}
+    for env_name in CASES:
+        ckpt = os.path.join(REF, 'pretrained', env_name, 'models', 'step_500000')
+        out[env_name] = {}
+        for net in ('cbf', 'actor'):
+            path = os.path.join(ckpt, f'{net}.pkl')
+            sd = torch.load(path, map_location='cpu')
+            assert all(v.dtype == torch.float32 for v in sd.values())
+            out[env_name][net] = dict(file_bytes=os.path.getsize(path), keys=[[k, list(v.shape)] for k, v in sd.items()],
+                                      metadata=getattr(sd, '_metadata', {}))
+    path = os.path.join(ROOT, 'tests', 'golden', 'pretrained_checkpoints.json')
+    with open(path, 'w') as f:
+        json.dump(out, f, indent=1)
+        f.write('\n')
+    print(f'{path}: {os.path.getsize(path)} B')
 
 
 if __name__ == '__main__':
-    main()
+    if sys.argv[1:] == ['manifest']:
+        checkpoint_manifest()
+    else:
+        main()

@@ -305,8 +305,10 @@ class _NoEvent:
 
 
 def install(monkeypatch, host_lib, jvp_host_lib=None):
-    """Route the product's C-ABI calls to a FakeDevice for the duration of a test.  Returns the FakeDevice."""
-    from gcbf_b200 import _C, native, ops
+    """Route the product's C-ABI calls to a FakeDevice for the duration of a test.  Returns the FakeDevice.  ops and jvp bind `call`
+    at import, so both are imported here before anything is patched and their bindings are patched (and restored) as well: a module
+    first imported under the patch would otherwise keep the fake for the rest of the session."""
+    from gcbf_b200 import _C, jvp, native, ops
     fd = FakeDevice(host_lib)
     fd.jvp_host = jvp_host_lib
     monkeypatch.setattr(torch.cuda, 'Event', _NoEvent)                    # ops.sn_power_iter_batched orders its iterations with events
@@ -331,6 +333,7 @@ def install(monkeypatch, host_lib, jvp_host_lib=None):
 
     monkeypatch.setattr(_C, 'call', call)
     monkeypatch.setattr(ops, 'call', call)
+    monkeypatch.setattr(jvp, 'call', call)
     monkeypatch.setattr(_C, 'require_cuda', lambda *t: None)
     monkeypatch.setattr(_C, 'stream', lambda: None)
     monkeypatch.setattr(native, 'fn', fn)

@@ -106,14 +106,26 @@ def test_state_dict_key_contract():
     assert act.state_dict()['feat_2_action.net.0.weight'].shape == (512, 1026)
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/pretrained'), reason='shipped checkpoints live in the reference checkout')
 @pytest.mark.parametrize('env_name', ['SimpleCar', 'DubinsCar', 'SimpleDrone'])
 def test_shipped_checkpoints_load_strictly(env_name, tmp_path):
-    """All six shipped checkpoint files (pretrained/<env>/models/step_500000/{cbf,actor}.pkl, SURVEY 8a row a13) load with
-    strict=True into the product modules through GCBF.load, also AFTER the parameters were re-homed into the flat bucket, and
-    GCBF.save writes files of the reference's size (no bucket-sized storages) that the oracle port reads back unchanged."""
+    """Checkpoints laid out as the six shipped files (pretrained/<env>/models/step_500000/{cbf,actor}.pkl, SURVEY 8a row a13:
+    key order, shapes and state-dict metadata from tests/golden/pretrained_checkpoints.json, seeded values in place of the
+    trained weights) load with strict=True into the product modules through GCBF.load, also AFTER the parameters were
+    re-homed into the flat bucket, and GCBF.save writes files of the shipped files' size (no bucket-sized storages) that
+    the oracle port reads back unchanged."""
+    import json
+    from collections import OrderedDict
+    from conftest import GOLDEN_DIR
     from gcbf_b200.synth import seeded_algo
-    ckpt = f'/root/reference/pretrained/{env_name}/models/step_500000'
+    with open(os.path.join(GOLDEN_DIR, 'pretrained_checkpoints.json')) as f:
+        layout = json.load(f)[env_name]
+    ckpt = str(tmp_path / 'step_500000')
+    os.makedirs(ckpt)
+    g = torch.Generator().manual_seed(0)
+    for net in ('cbf', 'actor'):
+        sd = OrderedDict((k, torch.randn(shape, generator=g)) for k, shape in layout[net]['keys'])
+        sd._metadata = OrderedDict(layout[net]['metadata'])
+        torch.save(sd, os.path.join(ckpt, f'{net}.pkl'))
     env, algo = seeded_algo(env_name, 16, torch.device('cpu'))
     algo._ensure_bucket()                               # parameters become views into the flat bucket
     algo.load(ckpt)
@@ -128,7 +140,7 @@ def test_shipped_checkpoints_load_strictly(env_name, tmp_path):
     algo.save(str(tmp_path))
     for f, want in (('cbf.pkl', want_c), ('actor.pkl', want_a)):
         size = os.path.getsize(tmp_path / f)
-        assert abs(size - os.path.getsize(os.path.join(ckpt, f))) < 65536, (f, size)      # not 2x: each file holds ONE net
+        assert abs(size - layout[f[:-4]]['file_bytes']) < 65536, (f, size)      # not 2x: each file holds ONE net
         back = torch.load(tmp_path / f, map_location='cpu')
         assert all(torch.equal(back[k], want[k]) for k in want)
 

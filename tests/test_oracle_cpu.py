@@ -1,21 +1,32 @@
 """CPU tests of the oracle (oracle/gcbf_oracle.py):
   1. against the committed golden fixtures (generated from the reference by oracle/make_golden.py);
-  2. against the live reference (oracle/ref_harness.py in a subprocess) when /root/reference is present;
-  3. semantic known-answer on the shipped pretrained checkpoints (when present).
+  2. bit for bit against stored runs of the reference's own train step and replay buffer (tests/golden/reference_runs.json);
+  3. semantic known-answer on the shipped pretrained checkpoints (when the reference checkout is present).
 """
+import hashlib
+import json
 import os
-import subprocess
-import sys
 
 import pytest
 import torch
 
 import gcbf_oracle as O
-from conftest import ROOT, digest_close, golden_cases, load_golden
+import ref_loader
+from conftest import GOLDEN_DIR, digest_close, golden_cases, load_golden
 from helpers import case_inputs, oracle_batch, sd_clone, seeded_algo
 
-REF = '/root/reference'
-has_ref = os.path.isdir(os.path.join(REF, 'gcbf'))
+PRETRAINED_CBF = os.path.join(ref_loader.REFERENCE_ROOT, 'pretrained', 'SimpleCar', 'models', 'step_500000', 'cbf.pkl')
+
+
+@pytest.fixture(autouse=True)
+def _fixture_threads():
+    """The seeded initialisation runs MKL's QR (orthogonal_), whose rounding depends on the number of intra-op threads: the port
+    reproduces the stored reference weights bit for bit only at the thread count the fixtures were made with."""
+    import make_golden
+    n = torch.get_num_threads()
+    torch.set_num_threads(make_golden.THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def _run_port(fix_like_meta, sb, n_steps):
@@ -82,32 +93,39 @@ def test_port_apply_matches_golden(case):
     assert torch.allclose(a, fix['apply_action'], rtol=1e-4, atol=1e-4), (a - fix['apply_action']).abs().max()
 
 
-@pytest.mark.skipif(not has_ref, reason='reference checkout not present (GPU box)')
+def _reference_runs():
+    with open(os.path.join(GOLDEN_DIR, 'reference_runs.json')) as f:
+        return json.load(f)
+
+
+def _sha256(t):
+    return hashlib.sha256(t.detach().cpu().contiguous().numpy().tobytes()).hexdigest()
+
+
 @pytest.mark.parametrize('cfg', [('SimpleCar', 12, 0, 2, 2.0), ('DubinsCar', 10, 3, 2, 2.0), ('SimpleDrone', 6, 6, 2, 1.0)])
-def test_port_matches_live_reference(cfg, tmp_path):
+def test_port_matches_live_reference(cfg):
+    """One train step of the port bit for bit against the reference's own (oracle/ref_harness.py, stored by
+    `oracle/make_golden.py live`): edge_index, h, u and every tensor of both post-step state dicts (by SHA-256)."""
     env_name, n, obs, graphs, area = cfg
-    out = tmp_path / 'ref.pt'
-    subprocess.check_call([sys.executable, os.path.join(ROOT, 'oracle', 'ref_harness.py'), '--env', env_name, '--n', str(n),
-                           '--obs', str(obs), '--graphs', str(graphs), '--area', str(area), '--seed', '5', '--steps', '1',
-                           '--out', str(out)], stderr=subprocess.DEVNULL)
-    ref = torch.load(out, weights_only=False)
+    ref = next(c for c in _reference_runs()['train_step'] if (c['env'], c['n'], c['obs'], c['graphs'], c['area']) == cfg)
     from gcbf_b200 import synth
-    sb = synth.make_states(env_name, n, obs, graphs, area, 5)
+    sb = synth.make_states(env_name, n, obs, graphs, area, ref['seed'])
     r = _run_port(dict(init_seed=0), sb, 1)
-    assert torch.equal(r['ob']['edge_index'], ref['edge_index'])
-    assert torch.equal(r['h'], ref['h_probe']) and torch.equal(r['u'], ref['u_probe'])
-    for k in ref['cbf_final']:
-        assert torch.equal(r['cbf'][k], ref['cbf_final'][k]), k
-    for k in ref['actor_final']:
-        assert torch.equal(r['actor'][k], ref['actor_final'][k]), k
+    assert torch.equal(r['ob']['edge_index'], torch.tensor(ref['edge_index'], dtype=r['ob']['edge_index'].dtype))
+    assert torch.equal(r['h'], torch.tensor(ref['h_probe'], dtype=torch.float32))
+    assert torch.equal(r['u'], torch.tensor(ref['u_probe'], dtype=torch.float32))
+    for got, want in ((r['cbf'], ref['cbf_final_sha256']), (r['actor'], ref['actor_final_sha256'])):
+        assert list(got) == list(want)
+        for k in want:
+            assert _sha256(got[k]) == want[k], k
 
 
-@pytest.mark.skipif(not has_ref, reason='pretrained checkpoints live in the reference checkout')
+@pytest.mark.skipif(not os.path.exists(PRETRAINED_CBF), reason="needs the reference checkout's trained SimpleCar checkpoint (49 MB)")
 def test_pretrained_semantic_known_answer():
     """The shipped SimpleCar CBF must separate colliding from well-separated agents when evaluated through the
     port's restatement of PyG's message ordering / attention (SURVEY section 4): a wrong gather order or softmax
     grouping destroys this."""
-    cbf = torch.load(os.path.join(REF, 'pretrained/SimpleCar/models/step_500000/cbf.pkl'), map_location='cpu')
+    cbf = torch.load(PRETRAINED_CBF, map_location='cpu')
     from gcbf_b200 import synth
     hs, safe, coll = [], [], []
     for seed in range(20):
@@ -163,39 +181,13 @@ def test_fp16x3_model_accuracy():
     assert ((rec - a.double()).abs() <= a.abs().double() * 2.0 ** -21 + a.abs().max().item() * 2.0 ** -39).all()
 
 
-@pytest.mark.skipif(not has_ref, reason='reference checkout not present (GPU box)')
-def test_buffer_sampling_matches_live_reference(tmp_path):
+def test_buffer_sampling_matches_live_reference():
     """The replay buffers' index semantics (append, safe / unsafe bookkeeping, merge, segment sampling and its consumption
-    of the host RNG streams) against the reference's OWN gcbf/algo/buffer.py, run in a subprocess on the shim."""
-    script = tmp_path / 'run_ref_buffer.py'
-    script.write_text(f"""
-import sys, json, random
-import numpy as np
-sys.path.insert(0, {os.path.join(ROOT, 'oracle')!r})
-import ref_loader
-ref_loader.load_reference()
-from gcbf.algo.buffer import Buffer
-buf, other = Buffer(), Buffer()
-for i in range(90):
-    buf.append(i, i % 4 != 0)
-for i in range(200, 230):
-    other.append(i, i % 3 == 0)
-out = []
-for seed, (n, m, bal) in enumerate([(12, 3, False), (16, 3, True), (7, 1, False), (20, 5, True)]):
-    np.random.seed(seed); random.seed(seed)
-    out.append(buf.sample(n, m, bal))
-buf.merge(other)
-np.random.seed(9); random.seed(9)
-out.append(buf.sample(24, 3, True))
-out.append([buf.size, buf.safe_data[-3:], buf.unsafe_data[-3:]])
-json.dump(out, open({str(tmp_path / 'out.json')!r}, 'w'))
-""")
-    subprocess.check_call([sys.executable, str(script)], stderr=subprocess.DEVNULL)
-    import json
+    of the host RNG streams) against the reference's OWN gcbf/algo/buffer.py (stored by `oracle/make_golden.py live`)."""
     import random
     import types
     import numpy as np
-    want = json.load(open(tmp_path / 'out.json'))
+    want = _reference_runs()['buffer_sampling']
     from gcbf_b200.algo.buffer import Buffer
     from gcbf_b200.algo.device_buffer import DeviceReplay
 
